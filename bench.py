@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  (CPU arm: the oracle port, all host threads)
+    python bench.py ... --dump-outputs DIR                   (also write what the last timed step returned, DIR/<name>.npy)
 
 One "step" = one env.step() of every env of this rank's shard = ONE k_hover_step launch (6 physics substeps,
 3 control ticks, reward / termination / observation fused; finished envs are reset by their own thread on the next
@@ -309,6 +310,39 @@ def dogfight_split_block(rank, world, dev, steps=40, arenas=8192):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def timed_step_outputs(env) -> dict:
+    """What env.step() returned for the batch of the last timed step, as float32 host arrays.  Above DUMP_LIMIT_BYTES only a
+    fixed, seeded sample of the envs is kept; `env_index` (float64) says which."""
+    import numpy as np
+
+    av = env.aviary
+    bits = av.info_bits.cpu().numpy()
+    out = {
+        "obs": av.obs.cpu().numpy(), "reward": av.reward.cpu().numpy(),
+        "terminated": av.term.cpu().numpy().astype(np.float32), "truncated": av.trunc.cpu().numpy().astype(np.float32),
+        "info_out_of_bounds": (bits & 1).astype(np.float32), "info_collision": ((bits >> 1) & 1).astype(np.float32),
+        "info_env_complete": ((bits >> 2) & 1).astype(np.float32),
+    }
+    n = av.num_drones
+    row_bytes = sum(a[0].nbytes for a in out.values()) + 8
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        out = {k: v[keep] for k, v in out.items()}
+        out["env_index"] = keep.astype(np.float64)
+    return out
+
+
+def write_outputs(directory: str, arrays: dict) -> None:
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -386,6 +420,8 @@ def run_ours(args, rank, local_rank, world):
     launches0 = sum(e.aviary.launch_count for e in rot)
     block_ms = [rotating_block(K, W + r * K) for r in range(R)]
     launches = (sum(e.aviary.launch_count for e in rot) - launches0) // R
+    # the later regions step these batches again: keep what the last timed step returned
+    dumped = timed_step_outputs(rot[(K - 1) % M]) if args.dump_outputs and rank == 0 else None
     # ---- region R (context): the same K env steps of the same batches as FUSED rollouts — pfb_env_rollout(16): 16 env steps per
     #      launch with the state in registers, actions drawn on device, every step's observations / rewards / flags written, spares
     #      topped up behind every launch (all inside the event pair); "synthetic random-action rollouts" in BASELINE.json's words
@@ -588,6 +624,8 @@ def run_ours(args, rank, local_rank, world):
             os._exit(0)
         dog.cancel()
     emit(split)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -608,6 +646,9 @@ def main():
     ap.add_argument("--batches", type=int, default=12,
                     help="independent 65 536-env batches stepped round-robin in the timed region (their working set exceeds the L2: every "
                          "launch finds its inputs in DRAM); 1 = one batch, L2-warm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (obs, reward, terminated, truncated, info flags; rank 0's "
+                         "shard under torchrun) as DIR/<name>.npy in float32; inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))

@@ -1,8 +1,8 @@
 """pfb_model_from_files (C-ABI, pyflyt_b200/csrc/pfb_model_files.cu): URDF + parameter YAML -> PfbModel without Python.
 Checked field by field against the Python table builder (pyflyt_b200/models/{urdf,tables}.py, itself checked against
 SURVEY.md A.2 in tests/test_models.py) on synthetic vehicles written here — rotated joint / inertial / collision frames,
-comments, a stray tail after </robot>, scalar and list PID gains — and, where the reference checkout is present (this
-container, not the GPU box), on the reference's own five vehicle directories."""
+comments, a stray tail after </robot>, scalar and list PID gains — and on the original PyFlyt's own five vehicle
+descriptions (URDF + YAML, stored unmodified under tests/golden/vehicles)."""
 import os
 
 import pytest
@@ -10,7 +10,7 @@ import pytest
 from pyflyt_b200._lib import PfbError
 from pyflyt_b200.models.tables import build_model, model_from_files, model_to_dict
 
-REF_MODELS = "/root/reference/PyFlyt/models/vehicles"
+REF_MODELS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "vehicles")
 
 
 def _link(name, mass, ixyz=(0, 0, 0), irpy=(0, 0, 0), inertia=(0, 0, 0, 0, 0, 0), collision=""):
@@ -220,8 +220,6 @@ def test_c_loader_equals_python_table_builder(tmp_path, kind, maker):
 @pytest.mark.parametrize("kind,name", [("quadx", "cf2x"), ("quadx", "primitive_drone"), ("fixedwing", "fixedwing"), ("fixedwing", "acrowing"),
                                        ("rocket", "rocket")])
 def test_c_loader_on_the_reference_vehicles(kind, name):
-    if not os.path.isdir(REF_MODELS):
-        pytest.skip("reference checkout not present (GPU box)")
     urdf, yml = os.path.join(REF_MODELS, name, f"{name}.urdf"), os.path.join(REF_MODELS, name, f"{name}.yaml")
     c = model_to_dict(model_from_files(kind, urdf, yml))
     _assert_same(model_to_dict(build_model(kind, name, model_dir=REF_MODELS)), c)  # the Python parser on the same files
