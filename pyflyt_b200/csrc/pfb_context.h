@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <type_traits>
 
 #include "../../include/pyflyt_b200.h"
 #include "pfb_fixedwing.cuh"
@@ -128,29 +129,103 @@ static inline StepPlan plan_step(PfbContext* h) {
   return p;
 }
 
-// ---- reset pipeline plumbing shared by the env kinds that keep spare post-reset states (DESIGN.md §4) ----------------
-// before step k: the rebuild of the spares consumed by step k - 2 must be complete (an env cannot finish again sooner)
-#define SPARE_BEFORE_STEP(h, s)                                                                          \
-  do {                                                                                                   \
-    if ((h)->d_spare && (h)->env.autoreset && (h)->step_seq >= 2)                                        \
-      CUDA_OK(cudaStreamWaitEvent((s), (h)->ev_spare[((h)->step_seq - 2) % 4], 0));                      \
-  } while (0)
-// after step k was launched on `s`: order the side stream behind it; the caller then launches the build-mode kernel on
-// (h)->side and calls SPARE_REBUILD_DONE
-#define SPARE_REBUILD_BEGIN(h, s)                              \
-  do {                                                         \
-    CUDA_OK(cudaEventRecord((h)->ev_step, (s)));               \
-    CUDA_OK(cudaStreamWaitEvent((h)->side, (h)->ev_step, 0));  \
-  } while (0)
-#define SPARE_REBUILD_DONE(h) CUDA_OK(cudaEventRecord((h)->ev_spare[(h)->step_seq % 4], (h)->side))
-// before a user reset rewrites the spares: the last rebuild must have finished
-#define SPARE_BEFORE_RESET(h, s)                                                                         \
-  do {                                                                                                   \
-    if ((h)->d_spare && (h)->step_seq > 0) CUDA_OK(cudaStreamWaitEvent((s), (h)->ev_spare[((h)->step_seq - 1) % 4], 0)); \
-  } while (0)
+// template argument MODE (QuadX flight mode) from a run-time value
+#define PFB_MODE_SWITCH(mode, BODY)                         \
+  switch (mode) {                                           \
+    case -1: { constexpr int MODE = -1; BODY; } break;      \
+    case 0: { constexpr int MODE = 0; BODY; } break;        \
+    case 1: { constexpr int MODE = 1; BODY; } break;        \
+    case 2: { constexpr int MODE = 2; BODY; } break;        \
+    case 3: { constexpr int MODE = 3; BODY; } break;        \
+    case 4: { constexpr int MODE = 4; BODY; } break;        \
+    case 5: { constexpr int MODE = 5; BODY; } break;        \
+    case 6: { constexpr int MODE = 6; BODY; } break;        \
+    case 7: { constexpr int MODE = 7; BODY; } break;        \
+    default: return fail("`mode` must be between -1 and 7, got %d", mode); \
+  }
 
 // pfb_lib.cu: a masked user reset on an autoreset handle removes the masked envs / arenas from the pending done list
 int pfb_drop_masked_done(PfbContext* h, const uint8_t* mask, cudaStream_t s);
+
+// ---- NEXT_STEP autoreset by tail CTAs with spare post-reset states (DESIGN.md §4): QuadX-Waypoints, Fixedwing-Waypoints,
+// Rocket-Landing and Dogfight.  The device half is pfb_tail_reset.cuh.
+// The step kernels' bookkeeping arguments.  Normal launch: tail CTAs reset the entries of (prev_count, prev_list), finished
+// envs are appended to (cur_count, cur_list), next_count is zeroed.  Build mode (build = 1, only tail CTAs): the spares of the
+// entries of prev_list are rebuilt for the following episode, or of every env when prev_list is null.  The spare records
+// themselves stay a separate __restrict__ kernel argument: the kernels read and write them next to the state tensor.
+struct TailArgs {
+  const int32_t* prev_count;
+  const int32_t* prev_list;
+  int32_t* cur_count;
+  int32_t* cur_list;
+  int32_t* next_count;
+  int spare_copy;  // a tail CTA may copy a valid spare (0: inline_reset, every warm-up runs inline)
+  int build;
+  int tail_blocks;
+  uint32_t step_seq;
+};
+
+// `launch(inject, randact, autoreset, grid, stream, spare, args)` launches the kind's step kernel with the spare records
+// (nullptr: every reset runs its warm-up inline); the three flags are
+// std::integral_constant<bool, ...> so that it can name the template instantiation.  Returns 0 or the result of fail().
+using TailFalse = std::false_type;
+using TailTrue = std::true_type;
+
+template <typename Launch>
+int tail_env_step(PfbContext* h, const float* noise, bool randact, cudaStream_t s, Launch&& launch) {
+  if (h->env.autoreset && noise) return fail("injected noise (parity mode) is only supported with autoreset = 0");
+  const StepPlan pl = plan_step(h);
+  float* spare = h->env.autoreset ? h->d_spare : nullptr;
+  // the rebuild of the spares consumed by step k - 2 must be complete before step k (an env cannot finish again sooner)
+  if (spare && h->step_seq >= 2) CUDA_OK(cudaStreamWaitEvent(s, h->ev_spare[(h->step_seq - 2) % 4], 0));
+  if (pl.prof) CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n], s));
+  TailArgs a{pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, pl.cnt_next, (spare && !h->env.inline_reset) ? 1 : 0, 0, pl.tail, pl.seq};
+  int e;
+  if (h->env.autoreset) e = randact ? launch(TailFalse{}, TailTrue{}, TailTrue{}, pl.grid, s, spare, a) : launch(TailFalse{}, TailFalse{}, TailTrue{}, pl.grid, s, spare, a);
+  else if (noise) e = launch(TailTrue{}, TailFalse{}, TailFalse{}, pl.grid, s, spare, a);
+  else e = randact ? launch(TailFalse{}, TailTrue{}, TailFalse{}, pl.grid, s, spare, a) : launch(TailFalse{}, TailFalse{}, TailFalse{}, pl.grid, s, spare, a);
+  if (e) return e;
+  LAUNCH_CHECK(h);
+  if (pl.prof) {
+    CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n + 1], s));
+    h->prof_n += 1;
+  }
+  if (spare) {  // rebuild the spares this launch consumed, on the side stream, ordered behind it, while the next launches run
+    CUDA_OK(cudaEventRecord(h->ev_step, s));
+    CUDA_OK(cudaStreamWaitEvent(h->side, h->ev_step, 0));
+    a.spare_copy = 0;
+    a.build = 1;
+    a.tail_blocks = h->sm_count;
+    if (int e2 = launch(TailFalse{}, TailFalse{}, TailTrue{}, h->sm_count, h->side, spare, a)) return e2;
+    LAUNCH_CHECK(h);
+    CUDA_OK(cudaEventRecord(h->ev_spare[h->step_seq % 4], h->side));
+  }
+  h->step_seq += 1;
+  return 0;
+}
+
+// `reset(seq, grid)` launches the kind's reset kernel with its episode number; `launch` is the kind's step launch as above
+template <typename Reset, typename Launch>
+int tail_env_reset(PfbContext* h, const uint8_t* mask, cudaStream_t s, Reset&& reset, Launch&& launch) {
+  const uint32_t seq = 0x80000000u | (uint32_t)h->reset_seq++;
+  const int g = grid_for(h->n);
+  float* spare = h->env.autoreset ? h->d_spare : nullptr;
+  if (spare) {
+    // the spares are rewritten below: the last rebuild must have finished
+    if (h->step_seq > 0) CUDA_OK(cudaStreamWaitEvent(s, h->ev_spare[(h->step_seq - 1) % 4], 0));
+    if (!mask) CUDA_OK(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(int32_t), s));  // a full reset empties the autoreset queues
+    else if (pfb_drop_masked_done(h, mask, s)) return -1;  // a masked one takes its envs out of the pending done list
+  }
+  if (int e = reset(seq, g)) return e;
+  LAUNCH_CHECK(h);
+  if (spare) {  // every env gets a fresh spare: the step kernel in build mode over all envs, same stream
+    const TailArgs a{nullptr, nullptr, nullptr, nullptr, nullptr, 0, 1, g, 0u};
+    if (int e = launch(TailFalse{}, TailFalse{}, TailTrue{}, g, s, spare, a)) return e;
+    LAUNCH_CHECK(h);
+  }
+  h->mode = 0;
+  return 0;
+}
 
 // fixedwing translation unit (pfb_fixedwing.cu)
 int fw_build_params(const PfbModel& m, const PfbEnvConfig* env, pfb::FixedwingParams& p, pfb::WaypointParams& w);

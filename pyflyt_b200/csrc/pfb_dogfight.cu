@@ -12,6 +12,7 @@
 
 #include "pfb_context.h"
 #include "pfb_noise.cuh"
+#include "pfb_tail_reset.cuh"
 
 using namespace pfb;
 
@@ -48,11 +49,11 @@ int df_build_params(const PfbEnvConfig* env, DogfightParams& d) {
 }
 int df_obs_dim(const PfbContext* h) { return 23 + 14 * (2 * h->df.team_size - 1); }
 
-// spare post-reset states (the QuadX-Hover reset pipeline, DESIGN.md §4): one env-major record of 160 floats per AGENT —
-// the FW_* / DF_* state words, received-hits counter, validity, flags, episode number, and the agent's first observation
-// (its past-action slots are patched when the spare is used: the action history survives resets)
-enum { DSP_HITS = FW_ROWS, DSP_VALID = FW_ROWS + 1, DSP_FLAGS = FW_ROWS + 2, DSP_EPISODE = FW_ROWS + 3, DSP_OBS = 64, DSP_ROWS = 160 };
-static_assert(FW_ROWS + 4 <= DSP_OBS && DSP_OBS + 23 + 14 * 3 <= DSP_ROWS, "spare record too small");
+// spare post-reset states (pfb_tail_reset.cuh): one env-major record of 160 floats per AGENT — the FW_* / DF_* state words,
+// the spare header, the received-hits counter and the agent's first observation (its past-action slots are patched when the
+// spare is used: the action history survives resets)
+enum { DSP_HITS = SpareHdr<FW_ROWS>::END, DSP_OBS = 64, DSP_ROWS = 160 };
+static_assert(DSP_HITS < DSP_OBS && DSP_OBS + 23 + 14 * 3 <= DSP_ROWS, "spare record too small");
 constexpr int kDfObsPast = 19;  // index of past_actions inside the observation (3 + 3 + 3 + 3 + 5 + 1 + 1)
 int df_spare_rows() { return DSP_ROWS; }
 
@@ -284,39 +285,27 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
               float* __restrict__ st, int32_t* __restrict__ ist, float* __restrict__ actions, const float* __restrict__ noise,
               float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ term, uint8_t* __restrict__ trunc,
               uint8_t* __restrict__ info, const float* __restrict__ start_pos, const float* __restrict__ start_orn,
-              const int32_t* __restrict__ prev_count, const int32_t* __restrict__ prev_list, int32_t* __restrict__ cur_count,
-              int32_t* __restrict__ cur_list, int32_t* __restrict__ next_count, float* __restrict__ spare, int spare_copy, int build,
-              int tail_blocks, uint32_t step_seq, int64_t N) {
+              float* __restrict__ spare, const __grid_constant__ TailArgs a, int64_t N) {
   __shared__ float smem[kBlock * kDfObsStride];
   __shared__ uint8_t row_skip[kBlock];
   constexpr int O = 23 + 14 * (A - 1);
-  const bool tail = AUTORESET && (int)blockIdx.x < tail_blocks;
-  const int64_t block_first = tail ? 0 : (int64_t)((int)blockIdx.x - (AUTORESET ? tail_blocks : 0)) * kBlock;
+  const uint32_t step_seq = a.step_seq;
+  // work items are whole arenas: a regular lane owns one agent; tail lanes stride over the done-arena list
+  TailWork sch = tail_schedule<A, AUTORESET>(a, N, threadIdx.x);  // N is a multiple of A: an arena is never cut
+  const bool tail = sch.tail;
   const int li = threadIdx.x % A;                 // agent index inside its arena
   const int base = (threadIdx.x & 31) - li;       // lane of the arena's agent 0
-  // work items are whole arenas: a regular lane owns one agent; tail lanes stride over the done-arena list
-  int t, t_end, t_stride;
-  if (tail) {
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !build) *next_count = 0;
-    t = (blockIdx.x * kBlock + threadIdx.x) / A;
-    t_end = prev_list ? *prev_count : (int)(N / A);  // build mode after a user reset: every arena
-    t_stride = tail_blocks * kBlock / A;
-  } else {
-    t = 0;
-    t_end = (block_first + threadIdx.x < N) ? 1 : 0;  // N is a multiple of A: an arena is never cut
-    t_stride = 1;
-  }
   bool skip = true;
   float* row = smem + threadIdx.x * kDfObsStride;
 #pragma unroll 1
-  for (;; t += t_stride) {
+  for (;; sch.t += sch.t_stride) {
     // whole arenas enter or leave together (t is arena-uniform), so every shuffle below names exactly the
     // lanes that are present
-    const bool go = t < t_end;
+    const bool go = sch.t < sch.t_end;
     unsigned lanes = __ballot_sync(0xffffffffu, go);
     if (lanes == 0u) break;
     if (!go) continue;
-    const int64_t i = tail ? (prev_list ? (int64_t)prev_list[t] : (int64_t)t * A) + li : block_first + threadIdx.x;
+    const int64_t i = tail_env<A>(a, sch, li);
     FixedwingRegs s;
     DfAgent ag;
     float rew_out = 0.0f;
@@ -326,15 +315,10 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
       // episode); build mode computes those spares; without usable spares the arena runs its warm-up inline.  The episode
       // number (arena-uniform: agent 0's) keys the spawn and the warm-up noise in all three cases.
       float* rec = spare ? spare + i * DSP_ROWS : nullptr;
-      uint32_t nseq = step_seq | 0x40000000u;
-      bool mine = false;
-      if (rec) {
-        nseq = __float_as_uint(rec[DSP_EPISODE]) + (build ? 1u : 0u);
-        mine = !build && spare_copy && rec[DSP_VALID] != 0.0f;
-      }
-      nseq = __shfl_sync(lanes, nseq, base);
+      const SpareProbe sp = spare_probe<FW_ROWS>(a, rec, nullptr, false);
+      const uint32_t nseq = __shfl_sync(lanes, sp.episode, base);
       const unsigned arena_mask = ((1u << A) - 1u) << base;
-      const bool hit = (__ballot_sync(lanes, mine) & arena_mask) == arena_mask;  // all of the arena's spares, or none
+      const bool hit = (__ballot_sync(lanes, sp.hit) & arena_mask) == arena_mask;  // all of the arena's spares, or none
       df_load_agent(st, ist, N, i, ag);  // current / past actions survive the reset, like the reference's arrays
       if (hit) {
         const float p0 = ag.past[0], p1 = ag.past[1], p2 = ag.past[2], p3 = ag.past[3];
@@ -343,22 +327,20 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
         df_load_agent(rec, ist, N, i, ag, 1, 0);
         ag.past[0] = p0; ag.past[1] = p1; ag.past[2] = p2; ag.past[3] = p3;
         ag.cur[0] = c0; ag.cur[1] = c1; ag.cur[2] = c2; ag.cur[3] = c3;
-        s.flags = __float_as_uint(rec[DSP_FLAGS]);
+        s.flags = __float_as_uint(rec[SpareHdr<FW_ROWS>::FLAGS]);
         for (int k = 0; k < O; ++k) row[k] = rec[DSP_OBS + k];
         row[kDfObsPast + 0] = p0; row[kDfObsPast + 1] = p1; row[kDfObsPast + 2] = p2; row[kDfObsPast + 3] = p3;
       }
       const unsigned inl = __ballot_sync(lanes, !hit);  // the arenas that run their warm-up here exchange among themselves
       if (!hit) {
-        if (build) rec[DSP_VALID] = 0.0f;  // invalid until the warm-up below is stored
+        if (a.build) spare_open<FW_ROWS>(rec, nullptr);
         df_reset_agent<A, false>(p, d, rng, start_pos, start_orn, nullptr, nseq, true, N, i, li, base, s, ag, row, inl);
       }
-      if (build) {
+      if (a.build) {
         fixedwing_store(rec, ist, N, i, s, false, 1, 0);
         df_store_agent(rec, ist, N, i, ag, 1, 0);
         for (int k = 0; k < O; ++k) rec[DSP_OBS + k] = row[k];
-        rec[DSP_FLAGS] = __uint_as_float(s.flags & ~(uint32_t)FLAG_AGENT_DONE);
-        rec[DSP_EPISODE] = __uint_as_float(nseq);
-        rec[DSP_VALID] = 1.0f;
+        spare_seal<FW_ROWS>(rec, s.flags & ~(uint32_t)FLAG_AGENT_DONE, nseq);
         continue;
       }
       s.flags &= ~(uint32_t)(FLAG_AGENT_DONE);
@@ -370,7 +352,7 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
       // carries this launch's fresh tag instead of AGENT_DONE (pfb_quadx.cuh, FLAG_FRESH*)
       const unsigned arena_mask = ((1u << A) - 1u) << base;
       const bool i_done = (s.flags & FLAG_AGENT_DONE) != 0;
-      const bool owned = (s.flags & (FLAG_AGENT_DONE | fresh_tag(step_seq))) != 0;
+      const bool owned = tail_owns(s.flags, FLAG_AGENT_DONE, step_seq);
       s.flags &= ~(uint32_t)FLAG_FRESH_ANY;
       const bool arena_done = (__ballot_sync(lanes, owned) & arena_mask) == arena_mask;
       lanes = __ballot_sync(lanes, !(AUTORESET && arena_done));
@@ -424,32 +406,12 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
         const unsigned arena_mask = ((1u << A) - 1u) << base;
         const unsigned done_lanes = __ballot_sync(lanes, (flags & FLAG_AGENT_DONE) != 0);
         const bool leader_done = (li == 0) && ((done_lanes & arena_mask) == arena_mask);
-        unsigned m = __ballot_sync(lanes, leader_done);
-        if (leader_done) {
-          int lane = threadIdx.x & 31;
-          int leader = __ffs(m) - 1;
-          int b0 = 0;
-          if (lane == leader) b0 = atomicAdd(cur_count, __popc(m));
-          b0 = __shfl_sync(m, b0, leader);
-          cur_list[b0 + __popc(m & ((1u << lane) - 1u))] = (int32_t)i;
-        }
+        append_done(a, sch, lanes, leader_done, i);
       }
     }
   }
   if (tail) return;
-  row_skip[threadIdx.x] = skip ? 1 : 0;
-  __syncthreads();
-  int64_t rows = N - block_first;
-  if (rows > kBlock) rows = kBlock;
-  const int total = (int)rows * O;
-  float* dst = obs + block_first * O;
-  const int dr = kBlock / O, dc = kBlock - dr * O;
-  int r = threadIdx.x / O, c = threadIdx.x - r * O;
-  for (int j = threadIdx.x; j < total; j += kBlock) {
-    if (!row_skip[r]) dst[j] = smem[r * kDfObsStride + c];
-    r += dr; c += dc;
-    if (c >= O) { c -= O; ++r; }
-  }
+  flush_obs_tile<kDfObsStride>(smem, row_skip, skip, obs, sch, O, N);
 }
 
 template <int A, bool INJECT>
@@ -482,77 +444,37 @@ __global__ void __launch_bounds__(kBlock)
 // ---------------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------------
+// k_df_step for tail_env_step / tail_env_reset
+static auto df_step_launch(PfbContext* h, float* actions, const float* noise) {
+  return [=](auto inject, auto randact, auto autoreset, int grid, cudaStream_t s, float* spare, const TailArgs& a) -> int {
+    constexpr bool I = decltype(inject)::value, R = decltype(randact)::value, AR = decltype(autoreset)::value;
+#define DF_ARGS h->fw, h->df, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, \
+                h->buf.info, h->buf.start_pos, h->buf.start_orn, spare, a, h->n
+    if (h->df.team_size == 1) k_df_step<2, I, R, AR><<<grid, kBlock, 0, s>>>(DF_ARGS);
+    else k_df_step<4, I, R, AR><<<grid, kBlock, 0, s>>>(DF_ARGS);
+#undef DF_ARGS
+    return 0;
+  };
+}
+
 int df_env_reset(PfbContext* h, const uint8_t* mask, const float* noise, cudaStream_t s) {
-  const uint32_t seq = 0x80000000u | (uint32_t)h->reset_seq++;
-  const int g = grid_for(h->n);
   const int A = 2 * h->df.team_size;
   if (h->n % A) return fail("the number of envs (%lld) must be a multiple of the arena size %d", (long long)h->n, A);
   const int rnd = h->env.randomize_drop;  // reused as "draw the spawn on device" for the dogfight
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  if (spare) {
-    SPARE_BEFORE_RESET(h, s);
-    if (!mask) CUDA_OK(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(int32_t), s));  // a full reset empties the autoreset queues
-    else if (pfb_drop_masked_done(h, mask, s)) return -1;  // a masked one takes its envs out of the pending done list
-  }
+  auto reset = [&](uint32_t seq, int g) -> int {
 #define DR_ARGS h->fw, h->df, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, mask, noise, h->buf.obs, seq, rnd, h->n
-  if (A == 2) { if (noise) k_df_reset<2, true><<<g, kBlock, 0, s>>>(DR_ARGS); else k_df_reset<2, false><<<g, kBlock, 0, s>>>(DR_ARGS); }
-  else { if (noise) k_df_reset<4, true><<<g, kBlock, 0, s>>>(DR_ARGS); else k_df_reset<4, false><<<g, kBlock, 0, s>>>(DR_ARGS); }
+    if (A == 2) { if (noise) k_df_reset<2, true><<<g, kBlock, 0, s>>>(DR_ARGS); else k_df_reset<2, false><<<g, kBlock, 0, s>>>(DR_ARGS); }
+    else { if (noise) k_df_reset<4, true><<<g, kBlock, 0, s>>>(DR_ARGS); else k_df_reset<4, false><<<g, kBlock, 0, s>>>(DR_ARGS); }
 #undef DR_ARGS
-  LAUNCH_CHECK(h);
-  if (spare) {  // every arena gets fresh spares: the step kernel in build mode over all arenas, same stream
-#define DB_ARGS h->fw, h->df, h->rng, h->buf.state, h->buf.istate, h->buf.setpoint, nullptr, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, \
-                h->buf.info, h->buf.start_pos, h->buf.start_orn, nullptr, nullptr, nullptr, nullptr, nullptr, spare, 0, 1, g, 0u, h->n
-    if (A == 2) k_df_step<2, false, false, true><<<g, kBlock, 0, s>>>(DB_ARGS);
-    else k_df_step<4, false, false, true><<<g, kBlock, 0, s>>>(DB_ARGS);
-#undef DB_ARGS
-    LAUNCH_CHECK(h);
-  }
-  h->mode = 0;
-  return 0;
+    return 0;
+  };
+  return tail_env_reset(h, mask, s, reset, df_step_launch(h, h->buf.setpoint, nullptr));
 }
 
 int df_env_step(PfbContext* h, float* actions, const float* noise, bool randact, cudaStream_t s) {
-  StepPlan pl = plan_step(h);
   const int A = 2 * h->df.team_size;
   if (h->n % A) return fail("the number of envs (%lld) must be a multiple of the arena size %d", (long long)h->n, A);
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  const int spare_copy = (spare && !h->env.inline_reset) ? 1 : 0;
-  SPARE_BEFORE_STEP(h, s);
-  if (pl.prof) CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n], s));
-#define DF_ARGS h->fw, h->df, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, \
-                h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, pl.cnt_next, spare, \
-                spare_copy, 0, pl.tail, pl.seq, h->n
-#define DF_LAUNCH(AA)                                                                                         \
-  if (h->env.autoreset) {                                                                                     \
-    if (noise) return fail("injected noise (parity mode) is only supported with autoreset = 0");              \
-    if (randact) k_df_step<AA, false, true, true><<<pl.grid, kBlock, 0, s>>>(DF_ARGS);                        \
-    else k_df_step<AA, false, false, true><<<pl.grid, kBlock, 0, s>>>(DF_ARGS);                               \
-  } else {                                                                                                    \
-    if (noise) k_df_step<AA, true, false, false><<<pl.grid, kBlock, 0, s>>>(DF_ARGS);                         \
-    else if (randact) k_df_step<AA, false, true, false><<<pl.grid, kBlock, 0, s>>>(DF_ARGS);                  \
-    else k_df_step<AA, false, false, false><<<pl.grid, kBlock, 0, s>>>(DF_ARGS);                              \
-  }
-  if (A == 2) { DF_LAUNCH(2) } else { DF_LAUNCH(4) }
-#undef DF_LAUNCH
-#undef DF_ARGS
-  LAUNCH_CHECK(h);
-  if (pl.prof) {
-    CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n + 1], s));
-    h->prof_n += 1;
-  }
-  if (spare) {  // rebuild the spares this launch consumed, on the side stream, while the next launches run
-    SPARE_REBUILD_BEGIN(h, s);
-#define DB_ARGS h->fw, h->df, h->rng, h->buf.state, h->buf.istate, actions, nullptr, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, \
-                h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, pl.cnt_next, spare, 0, 1, \
-                h->sm_count, pl.seq, h->n
-    if (A == 2) k_df_step<2, false, false, true><<<h->sm_count, kBlock, 0, h->side>>>(DB_ARGS);
-    else k_df_step<4, false, false, true><<<h->sm_count, kBlock, 0, h->side>>>(DB_ARGS);
-#undef DB_ARGS
-    LAUNCH_CHECK(h);
-    SPARE_REBUILD_DONE(h);
-  }
-  h->step_seq += 1;
-  return 0;
+  return tail_env_step(h, noise, randact, s, df_step_launch(h, actions, noise));
 }
 
 // ===================================================================================================

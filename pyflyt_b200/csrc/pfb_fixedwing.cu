@@ -6,6 +6,7 @@
 
 #include "pfb_context.h"
 #include "pfb_noise.cuh"
+#include "pfb_tail_reset.cuh"
 
 using namespace pfb;
 
@@ -183,85 +184,53 @@ __device__ __forceinline__ void wp_observation(const WaypointParams& w, const Fi
 
 // env.reset() for one env (fixedwing_waypoints_env.py:102-119, fixedwing_base_env.py:126-192); `pose` = the 6 start-pose
 // words the caller read (and, when building a spare, recorded), targets go to tb / ts
-template <bool INJECT, int L = 1>
+template <bool INJECT>
 __device__ __forceinline__ void wp_reset_env(const FixedwingParams& p, const WaypointParams& w, const RngParams& rng, const float* pose,
                                              const float* __restrict__ reset_targets, const float* __restrict__ noise, uint32_t seq,
-                                             int64_t N, int64_t i, float* __restrict__ tb, int64_t ts, FixedwingRegs& s, WpState& wp,
-                                             const SurfaceParams* __restrict__ surf = nullptr, int sub = 0, unsigned gmask = 0xffffffffu) {
+                                             int64_t N, int64_t i, float* __restrict__ tb, int64_t ts, FixedwingRegs& s, WpState& wp) {
   fixedwing_reset(p, s, pose[0], pose[1], pose[2], pose[3], pose[4], pose[5]);
-  if (sub == 0) {  // one lane of the aircraft's group installs the targets; the group re-converges before they are read
-    if (reset_targets) {
-      for (int k = 0; k < 3 * w.num_targets; ++k) tb[(int64_t)(FW_TARGETS + k) * ts] = reset_targets[(int64_t)i * 3 * w.num_targets + k];
-    } else {
-      wp_sample_targets(w, rng, i, seq, tb, ts);
-    }
+  if (reset_targets) {
+    for (int k = 0; k < 3 * w.num_targets; ++k) tb[(int64_t)(FW_TARGETS + k) * ts] = reset_targets[(int64_t)i * 3 * w.num_targets + k];
+  } else {
+    wp_sample_targets(w, rng, i, seq, tb, ts);
   }
-  if (L > 1) __syncwarp(gmask);
   wp.first = 0;
   wp.reached_now = false;
   wp.new_dist = INFINITY;
   wp_load_target0(tb, ts, wp);
   auto nz = make_noise<INJECT>(noise, N, i, rng, seq, TAG_RESET, p.noise_loc, p.ratio);
-  for (int k = 0; k < w.warmup_steps; ++k) {
-    if (L > 1) fixedwing_aviary_step_lanes<0, L>(p, surf, s, nz, sub, gmask);
-    else fixedwing_aviary_step<0>(p, s, nz);
-  }
-  if (L > 1) fixedwing_gather_act<L>(s, gmask);
+  for (int k = 0; k < w.warmup_steps; ++k) fixedwing_aviary_step<0>(p, s, nz);
   fixedwing_requantize(s);             // exactly what the state tensor / a spare record will hold
   (void)wp_update_distance(s, wp);     // end_reset -> compute_state
 }
 
-// ---- spare post-reset states: the QuadX-Hover reset pipeline (pfb_lib.cu, DESIGN.md §4) for this env.  A spare is an
-// env-major record of 64 floats: the FW_* state words INCLUDING the episode's targets and new_distance, then:
-enum { WSP_POSE = FW_ROWS, WSP_VALID = FW_ROWS + 6, WSP_FLAGS = FW_ROWS + 7, WSP_EPISODE = FW_ROWS + 8, WSP_ROWS = 64 };
-static_assert(FW_ROWS + 9 <= WSP_ROWS, "spare record too small");
+// spare post-reset states (pfb_tail_reset.cuh): an env-major record of 64 floats, the FW_* state words INCLUDING the
+// episode's targets and new_distance, then the spare header
+enum { WSP_ROWS = 64 };
+static_assert(SpareHdr<FW_ROWS>::END <= WSP_ROWS, "spare record too small");
 
-// L = lanes per aircraft (1: one thread per env; 4: pfb_fixedwing.cuh "L lanes per aircraft"): a CTA (one warp) owns kBlock / L envs
-#ifndef PFB_FW_ROLLED
-#define PFB_FW_ROLLED 0
-#endif
-constexpr bool kFwRolled = PFB_FW_ROLLED != 0;  // A/B knob: the step loop runs the surfaces through one rolled copy (instruction-cache footprint)
-template <bool INJECT, bool RANDACT, bool AUTORESET, int L>
+// One thread per aircraft.  Splitting the five lifting surfaces over L lanes per aircraft was measured slower on B200 (16 384
+// envs, L2 flushed, us per env step: L = 1: 37.5, L = 2: 39.3, L = 4: 41.8, L = 8: 58.6): the surfaces are only ~55 % of a
+// substep's instructions, the rest is replicated in every lane of a group (DESIGN.md §9).
+
+template <bool INJECT, bool RANDACT, bool AUTORESET>
 __global__ void __launch_bounds__(kBlock, kAeroBlocks)
     k_fwwp_step(const __grid_constant__ FixedwingParams p, const __grid_constant__ WaypointParams w,
                 const __grid_constant__ RngParams rng, float* __restrict__ st, int32_t* __restrict__ ist,
                 float* __restrict__ actions, const float* __restrict__ noise, float* __restrict__ obs, float* __restrict__ reward,
                 uint8_t* __restrict__ term, uint8_t* __restrict__ trunc, uint8_t* __restrict__ info,
-                const float* __restrict__ start_pos, const float* __restrict__ start_orn, const int32_t* __restrict__ prev_count,
-                const int32_t* __restrict__ prev_list, int32_t* __restrict__ cur_count, int32_t* __restrict__ cur_list,
-                int32_t* __restrict__ next_count, float* __restrict__ spare, int spare_copy, int build, int tail_blocks,
-                uint32_t step_seq, int64_t N) {
-  constexpr int EPB = kBlock / L;  // envs per CTA
-  __shared__ float smem[EPB * kWpObsStride];
-  __shared__ uint8_t row_skip[EPB];
-  __shared__ SurfaceParams ssurf[kMaxSurfaces];  // per-model coefficient rows: lane `sub` of a group reads the row of ITS surface
-  const int sub = L > 1 ? (int)(threadIdx.x % L) : 0;   // lane within the aircraft's group
-  const int slot = L > 1 ? (int)(threadIdx.x / L) : (int)threadIdx.x;  // env within the CTA
-  const unsigned gmask = L > 1 ? (((1u << L) - 1u) << (threadIdx.x & ~(L - 1))) : 0xffffffffu;
-  if (L > 1 || kFwRolled) {
-    for (int j = threadIdx.x; j < (int)(sizeof(SurfaceParams) / 4) * kMaxSurfaces; j += kBlock)
-      reinterpret_cast<float*>(ssurf)[j] = reinterpret_cast<const float*>(p.surf)[j];
-    __syncthreads();
-  }
+                const float* __restrict__ start_pos, const float* __restrict__ start_orn, float* __restrict__ spare, const __grid_constant__ TailArgs a, int64_t N) {
+  __shared__ float smem[kBlock * kWpObsStride];
+  __shared__ uint8_t row_skip[kBlock];
   const int O = (w.angle_representation == 0 ? 22 : 23) + 3 * w.num_targets;
-  const bool tail = AUTORESET && (int)blockIdx.x < tail_blocks;
-  const int64_t block_first = tail ? 0 : (int64_t)((int)blockIdx.x - (AUTORESET ? tail_blocks : 0)) * EPB;
-  int t, t_end, t_stride;
-  if (tail) {
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !build) *next_count = 0;
-    t = blockIdx.x * EPB + slot;
-    t_end = prev_list ? *prev_count : (int)N;  // build mode after a user reset: every env
-    t_stride = tail_blocks * EPB;
-  } else {
-    t = 0;
-    t_end = (block_first + slot < N) ? 1 : 0;
-    t_stride = 1;
-  }
+  const uint32_t step_seq = a.step_seq;
+  TailWork sch = tail_schedule<1, AUTORESET>(a, N, threadIdx.x);
+  const bool tail = sch.tail;
   bool skip = true;
-  float* row = smem + slot * kWpObsStride;
+  float* row = smem + threadIdx.x * kWpObsStride;
 #pragma unroll 1
-  for (; t < t_end; t += t_stride) {
-    const int64_t i = tail ? (prev_list ? (int64_t)prev_list[t] : (int64_t)t) : block_first + slot;
+  for (; sch.t < sch.t_end; sch.t += sch.t_stride) {
+    const int64_t i = tail_env<1>(a, sch, 0);
     FixedwingRegs s;
     WpState wp;
     float act[4] = {0.f, 0.f, 0.f, 0.f};
@@ -273,58 +242,42 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
       // env.reset(): normally a copy of the env's spare (state, targets, new_distance of the NEXT episode); build mode
       // computes that spare; without a usable spare the warm-up runs inline with the same episode number
       float* rec = spare ? spare + i * WSP_ROWS : nullptr;
-      uint32_t nseq = step_seq | 0x40000000u;
-      bool hit = false;
       float pose[6];
 #pragma unroll
       for (int k = 0; k < 3; ++k) { pose[k] = start_pos[3 * i + k]; pose[3 + k] = start_orn[3 * i + k]; }
-      if (rec) {
-        nseq = __float_as_uint(rec[WSP_EPISODE]) + (build ? 1u : 0u);
-        hit = !build && spare_copy && rec[WSP_VALID] != 0.0f;
-#pragma unroll
-        for (int k = 0; k < 6; ++k) hit = hit && (rec[WSP_POSE + k] == pose[k]);
-      }
-      if (hit) {
+      const SpareProbe sp = spare_probe<FW_ROWS>(a, rec, pose, true);
+      if (sp.hit) {
         fixedwing_load(rec, ist, N, i, s, 1, 0);
-        s.flags = __float_as_uint(rec[WSP_FLAGS]);
-        if (sub == 0)
-          for (int k = 0; k < 3 * w.num_targets; ++k) tb[(int64_t)(FW_TARGETS + k) * ts] = rec[FW_TARGETS + k];
+        s.flags = __float_as_uint(rec[SpareHdr<FW_ROWS>::FLAGS]);
+        for (int k = 0; k < 3 * w.num_targets; ++k) tb[(int64_t)(FW_TARGETS + k) * ts] = rec[FW_TARGETS + k];
         wp.first = 0;
         wp.reached_now = false;
         wp.new_dist = rec[FW_DIST];
       } else {
-        if (build) {
-          if (sub == 0) {
-            rec[WSP_VALID] = 0.0f;  // invalid until the warm-up below is stored
-#pragma unroll
-            for (int k = 0; k < 6; ++k) rec[WSP_POSE + k] = pose[k];
-          }
+        if (a.build) {
+          spare_open<FW_ROWS>(rec, pose);
           tb = rec;
           ts = 1;
         }
-        wp_reset_env<false, L>(p, w, rng, pose, nullptr, nullptr, nseq, N, i, tb, ts, s, wp, ssurf, sub, gmask);
+        wp_reset_env<false>(p, w, rng, pose, nullptr, nullptr, sp.episode, N, i, tb, ts, s, wp);
       }
-      if (build) {
-        if (sub == 0) {
-          fixedwing_store(rec, ist, N, i, s, false, 1, 0);
-          rec[FW_DIST] = wp.new_dist;
-          rec[WSP_FLAGS] = __uint_as_float(s.flags);
-          rec[WSP_EPISODE] = __uint_as_float(nseq);
-          rec[WSP_VALID] = 1.0f;
-        }
+      if (a.build) {
+        fixedwing_store(rec, ist, N, i, s, false, 1, 0);
+        rec[FW_DIST] = wp.new_dist;
+        spare_seal<FW_ROWS>(rec, s.flags, sp.episode);
         continue;
       }
       s.flags |= fresh_tag(step_seq);
     } else {
       fixedwing_load(st, ist, N, i, s);
-      if (AUTORESET && (s.flags & (FLAG_TERM | FLAG_TRUNC | fresh_tag(step_seq)))) continue;  // a tail CTA owns this env
+      if (AUTORESET && tail_owns(s.flags, FLAG_TERM | FLAG_TRUNC, step_seq)) continue;
       s.flags &= ~(uint32_t)FLAG_FRESH_ANY;
       if (RANDACT) {
         uint64_t g = ((uint64_t)rng.env_offset_hi << 32 | rng.env_offset_lo) + (uint64_t)i;
         U4 r = philox4x32_10(U4{(uint32_t)g, (uint32_t)(g >> 32), step_seq, (uint32_t)TAG_ACTION << 24}, rng.k0, rng.k1);
         act[0] = 2.0f * u32_to_unit_open(r.x) - 1.0f; act[1] = 2.0f * u32_to_unit_open(r.y) - 1.0f;
         act[2] = 2.0f * u32_to_unit_open(r.z) - 1.0f; act[3] = 2.0f * u32_to_unit_open(r.w) - 1.0f;
-        if (sub == 0) reinterpret_cast<float4*>(actions)[i] = make_float4(act[0], act[1], act[2], act[3]);
+        reinterpret_cast<float4*>(actions)[i] = make_float4(act[0], act[1], act[2], act[3]);
       } else {
         float4 a4 = __ldg(reinterpret_cast<const float4*>(actions) + i);
         act[0] = a4.x; act[1] = a4.y; act[2] = a4.z; act[3] = a4.w;
@@ -342,66 +295,36 @@ __global__ void __launch_bounds__(kBlock, kAeroBlocks)
 #pragma unroll 1
       for (int k = 0; k < w.env_step_ratio; ++k) {
         if (s.flags & (FLAG_TERM | FLAG_TRUNC)) break;
-        if (L > 1) fixedwing_aviary_step_lanes<0, L>(p, ssurf, s, nz, sub, gmask);
-        else if (kFwRolled) fixedwing_aviary_step_lanes<0, 1>(p, ssurf, s, nz, 0, 0xffffffffu);  // experiment: ONE rolled copy of the surface code
-        else if (full) fixedwing_aviary_step<0, true>(p, s, nz);
+        if (full) fixedwing_aviary_step<0, true>(p, s, nz);
         else fixedwing_aviary_step<0>(p, s, nz);
         float old = wp_update_distance(s, wp);
         wp_term_trunc_reward(w, s, wp, old, step_count, rew, tb, ts);
       }
       step_count += 1;
-      if (L > 1) fixedwing_gather_act<L>(s, gmask);
     }
     // the reference builds the observation in compute_state, BEFORE compute_term_trunc_reward advances the
     // target list: a target reached on the last Aviary step is still the head of the reported list
-    if (sub == 0) {  // one lane of the group writes the env's outputs
-      wp_observation(w, s, act, wp.first - (wp.reached_now ? 1 : 0), tb, ts, row);
-      fixedwing_store(st, ist, N, i, s);
-      st[(int64_t)FW_DIST * N + i] = wp.new_dist;
-      ist[(int64_t)FI_STEP * N + i] = step_count;
-      ist[(int64_t)FI_NTARGETS * N + i] = wp.first;
-      reward[i] = rew;
-      term[i] = (s.flags & FLAG_TERM) ? 1 : 0;
-      trunc[i] = (s.flags & FLAG_TRUNC) ? 1 : 0;
-      if (info)
-        info[i] = (uint8_t)(((s.flags & FLAG_OOB) ? 1 : 0) | ((s.flags & FLAG_COLLISION) ? 2 : 0) | ((s.flags & FLAG_ENV_COMPLETE) ? 4 : 0) |
-                            (wp.first << 3));
-    }
+    wp_observation(w, s, act, wp.first - (wp.reached_now ? 1 : 0), tb, ts, row);
+    fixedwing_store(st, ist, N, i, s);
+    st[(int64_t)FW_DIST * N + i] = wp.new_dist;
+    ist[(int64_t)FI_STEP * N + i] = step_count;
+    ist[(int64_t)FI_NTARGETS * N + i] = wp.first;
+    reward[i] = rew;
+    term[i] = (s.flags & FLAG_TERM) ? 1 : 0;
+    trunc[i] = (s.flags & FLAG_TRUNC) ? 1 : 0;
+    if (info)
+      info[i] = (uint8_t)(((s.flags & FLAG_OOB) ? 1 : 0) | ((s.flags & FLAG_COLLISION) ? 2 : 0) | ((s.flags & FLAG_ENV_COMPLETE) ? 4 : 0) |
+                          (wp.first << 3));
     if (tail) {
-      if (sub == 0) {
-        float* dst = obs + i * O;
-        for (int k = 0; k < O; ++k) dst[k] = row[k];
-      }
+      float* dst = obs + i * O;
+      for (int k = 0; k < O; ++k) dst[k] = row[k];
     } else {
       skip = false;
-      if (AUTORESET) {
-        bool done = sub == 0 && (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0;
-        unsigned m = __ballot_sync(__activemask(), done);
-        if (done) {
-          int lane = threadIdx.x & 31;
-          int leader = __ffs(m) - 1;
-          int base = 0;
-          if (lane == leader) base = atomicAdd(cur_count, __popc(m));
-          base = __shfl_sync(m, base, leader);
-          cur_list[base + __popc(m & ((1u << lane) - 1u))] = (int32_t)i;
-        }
-      }
+      if (AUTORESET) append_done(a, sch, __activemask(), (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0, i);
     }
   }
   if (tail) return;
-  if (sub == 0) row_skip[slot] = skip ? 1 : 0;
-  __syncthreads();
-  int64_t rows = N - block_first;
-  if (rows > EPB) rows = EPB;
-  const int total = (int)rows * O;
-  float* dst = obs + block_first * O;
-  const int dr = kBlock / O, dc = kBlock - dr * O;
-  int r = threadIdx.x / O, c = threadIdx.x - r * O;
-  for (int j = threadIdx.x; j < total; j += kBlock) {
-    if (!row_skip[r]) dst[j] = smem[r * kWpObsStride + c];
-    r += dr; c += dc;
-    if (c >= O) { c -= O; ++r; }
-  }
+  flush_obs_tile<kWpObsStride>(smem, row_skip, skip, obs, sch, O, N);
 }
 
 template <bool INJECT>
@@ -433,17 +356,6 @@ __global__ void __launch_bounds__(kBlock)
 // ---------------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------------
-// Lanes per aircraft in the Fixedwing-Waypoints step.  MEASURED on B200 (16 384 envs, L2 flushed, us per env step): L = 1: 37.5,
-// L = 2: 39.3, L = 4: 41.8, L = 8: 58.6 — splitting the five lifting surfaces over lanes does NOT pay: the surfaces are only
-// ~55 % of a substep's instructions; the Newton-Euler solve, the integrator and update_state are replicated in every lane of a
-// group, so 4x more warps carry 0.7x the instructions each (2.8x the issue work) for a 3x better issue rate.  Default 1; the
-// multi-lane path stays compiled behind -DPFB_FW_LANES=n as the record of the experiment (DESIGN.md 9).
-#ifndef PFB_FW_LANES
-#define PFB_FW_LANES 1
-#endif
-constexpr int kFwLanes = PFB_FW_LANES;
-static_assert(kFwLanes == 1 || kFwLanes == 2 || kFwLanes == 4 || kFwLanes == 8, "lanes per aircraft");
-
 int fw_reset(PfbContext* h, const uint8_t* mask, cudaStream_t s) {
   k_fw_reset<<<grid_for(h->n), kBlock, 0, s>>>(h->fw, h->buf.state, h->buf.istate, h->buf.setpoint, h->buf.start_pos,
                                                h->buf.start_orn, mask, fw_setpoint_dim(h), h->n);
@@ -483,69 +395,29 @@ int fw_observe(PfbContext* h, cudaStream_t s) {
   return 0;
 }
 
+// k_fwwp_step for tail_env_step / tail_env_reset
+static auto fw_step_launch(PfbContext* h, float* actions, const float* noise) {
+  return [=](auto inject, auto randact, auto autoreset, int grid, cudaStream_t s, float* spare, const TailArgs& a) -> int {
+    k_fwwp_step<decltype(inject)::value, decltype(randact)::value, decltype(autoreset)::value><<<grid, kBlock, 0, s>>>(
+        h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info,
+        h->buf.start_pos, h->buf.start_orn, spare, a, h->n);
+    return 0;
+  };
+}
+
 int fw_env_reset(PfbContext* h, const uint8_t* mask, const float* noise, cudaStream_t s) {
-  const uint32_t seq = 0x80000000u | (uint32_t)h->reset_seq++;
-  const int g = grid_for(h->n);
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  if (spare) {
-    SPARE_BEFORE_RESET(h, s);
-    if (!mask) CUDA_OK(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(int32_t), s));  // a full reset empties the autoreset queues
-    else if (pfb_drop_masked_done(h, mask, s)) return -1;  // a masked one takes its envs out of the pending done list
-  }
-  if (noise)
-    k_fwwp_reset<true><<<g, kBlock, 0, s>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn,
-                                            h->buf.reset_targets, mask, noise, h->buf.obs, seq, h->n);
-  else
-    k_fwwp_reset<false><<<g, kBlock, 0, s>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn,
-                                             h->buf.reset_targets, mask, nullptr, h->buf.obs, seq, h->n);
-  LAUNCH_CHECK(h);
-  if (spare) {  // every env gets a fresh spare: the step kernel in build mode over all envs, same stream
-    k_fwwp_step<false, false, true, kFwLanes><<<(g * kFwLanes), kBlock, 0, s>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, h->buf.setpoint, nullptr, h->buf.obs,
-                                                         h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn,
-                                                         nullptr, nullptr, nullptr, nullptr, nullptr, spare, 0, 1, g * kFwLanes, 0u, h->n);
-    LAUNCH_CHECK(h);
-  }
-  h->mode = 0;
-  return 0;
+  auto reset = [&](uint32_t seq, int g) -> int {
+    if (noise)
+      k_fwwp_reset<true><<<g, kBlock, 0, s>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn,
+                                              h->buf.reset_targets, mask, noise, h->buf.obs, seq, h->n);
+    else
+      k_fwwp_reset<false><<<g, kBlock, 0, s>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn,
+                                               h->buf.reset_targets, mask, nullptr, h->buf.obs, seq, h->n);
+    return 0;
+  };
+  return tail_env_reset(h, mask, s, reset, fw_step_launch(h, h->buf.setpoint, nullptr));
 }
 
 int fw_env_step(PfbContext* h, float* actions, const float* noise, bool randact, cudaStream_t s) {
-  StepPlan pl = plan_step(h);
-  // kFwLanes lanes per aircraft: a CTA (one warp) owns kBlock / kFwLanes envs
-  const int env_ctas = (int)((h->n + (kBlock / kFwLanes) - 1) / (kBlock / kFwLanes));
-  if (pl.tail > env_ctas) pl.tail = env_ctas;
-  pl.grid = env_ctas + pl.tail;
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  const int spare_copy = (spare && !h->env.inline_reset) ? 1 : 0;
-  SPARE_BEFORE_STEP(h, s);
-  if (pl.prof) CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n], s));
-#define WP_ARGS h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, \
-                h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, \
-                pl.cnt_next, spare, spare_copy, 0, pl.tail, pl.seq, h->n
-  if (h->env.autoreset) {
-    if (noise) return fail("injected noise (parity mode) is only supported with autoreset = 0");
-    if (randact) k_fwwp_step<false, true, true, kFwLanes><<<pl.grid, kBlock, 0, s>>>(WP_ARGS);
-    else k_fwwp_step<false, false, true, kFwLanes><<<pl.grid, kBlock, 0, s>>>(WP_ARGS);
-  } else {
-    if (noise) k_fwwp_step<true, false, false, kFwLanes><<<pl.grid, kBlock, 0, s>>>(WP_ARGS);
-    else if (randact) k_fwwp_step<false, true, false, kFwLanes><<<pl.grid, kBlock, 0, s>>>(WP_ARGS);
-    else k_fwwp_step<false, false, false, kFwLanes><<<pl.grid, kBlock, 0, s>>>(WP_ARGS);
-  }
-#undef WP_ARGS
-  LAUNCH_CHECK(h);
-  if (pl.prof) {
-    CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n + 1], s));
-    h->prof_n += 1;
-  }
-  if (spare) {  // rebuild the spares this launch consumed, on the side stream, while the next launches run
-    SPARE_REBUILD_BEGIN(h, s);
-    k_fwwp_step<false, false, true, kFwLanes><<<h->sm_count, kBlock, 0, h->side>>>(h->fw, h->wp, h->rng, h->buf.state, h->buf.istate, actions, nullptr,
-                                                                                   h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info,
-                                                                                   h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur,
-                                                                                   pl.list_cur, pl.cnt_next, spare, 0, 1, h->sm_count, pl.seq, h->n);
-    LAUNCH_CHECK(h);
-    SPARE_REBUILD_DONE(h);
-  }
-  h->step_seq += 1;
-  return 0;
+  return tail_env_step(h, noise, randact, s, fw_step_launch(h, actions, noise));
 }

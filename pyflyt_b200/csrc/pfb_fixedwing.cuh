@@ -333,75 +333,6 @@ PFB_HD void fixedwing_substep(const FixedwingParams& p, FixedwingRegs& s, const 
   body_update_state(s);
 }
 
-#if defined(__CUDACC__)
-// ---- L lanes per aircraft (the 16 384-env configs are latency-bound at one thread per env: < 1 warp per scheduler and a
-// 14 KB unrolled substep that misses the instruction cache on every iteration).  The L lanes of a group hold the same
-// rigid-body state; the lifting surfaces are dealt round-robin to the lanes (surface i -> lane i % L, pass i / L) and run
-// through ONE rolled copy of the surface code with per-lane coefficient rows from shared memory; the partial force / torque
-// sums are combined with a __shfl_xor butterfly (commutative adds: every lane ends up with the same bits), and the motor,
-// contact test, Newton-Euler step and update_state are replicated.  s.act[i] is current only on the owner lane of surface i
-// until fixedwing_gather_act() runs (once per env step, before the observation / the stores).
-PFB_HD float fw_sel5(const float* a, int i) { return i == 0 ? a[0] : (i == 1 ? a[1] : (i == 2 ? a[2] : (i == 3 ? a[3] : a[4]))); }
-template <int L>
-__device__ __forceinline__ void fixedwing_substep_lanes(const FixedwingParams& p, const SurfaceParams* __restrict__ surf, FixedwingRegs& s,
-                                                        const float* cmd, float xi, int sub, unsigned gmask) {
-  Vec3 F = Vec3{0.f, 0.f, 0.f}, T = Vec3{0.f, 0.f, 0.f};
-  const Vec3 w = Vec3{s.wx, s.wy, s.wz};
-  const bool windy = p.wind.kind != 0;
-  WindCtx wc = WindCtx{Vec3{0.f, 0.f, 0.f}, 0.f, 0.f, 0.f, 0.f};
-  if (windy) wc = wind_ctx(p.wind, (float)s.pz, (float)s.R.m00, (float)s.R.m01, (float)s.R.m02, (float)s.R.m10, (float)s.R.m11, (float)s.R.m12,
-                           (float)s.R.m20, (float)s.R.m21, (float)s.R.m22);
-  constexpr int kPasses = (kMaxSurfaces + L - 1) / L;
-#pragma unroll 1
-  for (int pass = 0; pass < kPasses; ++pass) {
-    const int i = pass * L + sub;
-    if (i < p.n_surfaces) {
-      float a = fw_sel5(s.act, i);
-      surface_force(surf[i], a, fw_sel5(cmd, i), s.vb, w, F, T, windy ? &p.wind : nullptr, &wc);
-#pragma unroll
-      for (int k = 0; k < kMaxSurfaces; ++k) s.act[k] = (i == k) ? a : s.act[k];
-    }
-  }
-#pragma unroll
-  for (int m = 1; m < L; m <<= 1) {
-    // gmask = the L lanes of this aircraft: groups of one warp may sit in different iterations of the caller's loops
-    F.x += __shfl_xor_sync(gmask, F.x, m); F.y += __shfl_xor_sync(gmask, F.y, m); F.z += __shfl_xor_sync(gmask, F.z, m);
-    T.x += __shfl_xor_sync(gmask, T.x, m); T.y += __shfl_xor_sync(gmask, T.y, m); T.z += __shfl_xor_sync(gmask, T.z, m);
-  }
-  {  // motor (motors.py:130-155), replicated
-    float t = s.thr;
-    t = fmaf(p.motor_lag, cmd[5] - t, t);
-    t = fmaf(xi * p.noise_ratio, t, t);
-    s.thr = t;
-    float a = t * fabsf(t);
-    Vec3 Fm = Vec3{p.thrust_k * a, 0.0f, 0.0f};
-    F = F + Fm;
-    T = T + cross(Vec3{p.motor_r[0], p.motor_r[1], p.motor_r[2]}, Fm) + Vec3{p.torque_k * a, 0.0f, 0.0f};
-  }
-  const bool c = ground_contact(p.contact, (float)s.pz, (float)s.R.m20, (float)s.R.m21, (float)s.R.m22);
-  s.flags = (s.flags & ~(uint32_t)FLAG_CONTACT_PREV) | (c ? (FLAG_CONTACT_PREV | FLAG_CONTACT_ARRAY) : 0u);
-  rigid_step(p.rb, p.gravity, p.dt, p.vmax, s, F, T);
-  body_update_state(s);
-}
-template <int MODE, int L, typename NoiseFn>
-__device__ __forceinline__ void fixedwing_aviary_step_lanes(const FixedwingParams& p, const SurfaceParams* __restrict__ surf, FixedwingRegs& s,
-                                                            NoiseFn& noise, int sub, unsigned gmask) {
-  s.flags &= ~(uint32_t)FLAG_CONTACT_ARRAY;
-  noise.begin_step();
-  float cmd[6];
-  fixedwing_command<MODE>(s, cmd);
-#pragma unroll 1
-  for (int u = 0; u < p.ratio; ++u) fixedwing_substep_lanes<L>(p, surf, s, cmd, noise.get(u), sub, gmask);
-}
-// every lane of a group gets the current actuation of every surface from its owner lane
-template <int L>
-__device__ __forceinline__ void fixedwing_gather_act(FixedwingRegs& s, unsigned gmask) {
-  const int lane = threadIdx.x & 31;
-#pragma unroll
-  for (int k = 0; k < kMaxSurfaces; ++k) s.act[k] = __shfl_sync(gmask, s.act[k], (lane & ~(L - 1)) | (k % L));
-}
-#endif
-
 template <int MODE, bool FULL = false, typename NoiseFn>
 PFB_HD void fixedwing_aviary_step(const FixedwingParams& p, FixedwingRegs& s, NoiseFn& noise) {
   s.flags &= ~(uint32_t)FLAG_CONTACT_ARRAY;

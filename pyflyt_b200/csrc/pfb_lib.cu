@@ -856,20 +856,6 @@ int pfb_drop_masked_done(PfbContext* h, const uint8_t* mask, cudaStream_t s) {
 // ---------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------
-#define PFB_MODE_SWITCH(mode, BODY)                         \
-  switch (mode) {                                           \
-    case -1: { constexpr int MODE = -1; BODY; } break;      \
-    case 0: { constexpr int MODE = 0; BODY; } break;        \
-    case 1: { constexpr int MODE = 1; BODY; } break;        \
-    case 2: { constexpr int MODE = 2; BODY; } break;        \
-    case 3: { constexpr int MODE = 3; BODY; } break;        \
-    case 4: { constexpr int MODE = 4; BODY; } break;        \
-    case 5: { constexpr int MODE = 5; BODY; } break;        \
-    case 6: { constexpr int MODE = 6; BODY; } break;        \
-    case 7: { constexpr int MODE = 7; BODY; } break;        \
-    default: return fail("`mode` must be between -1 and 7, got %d", mode); \
-  }
-
 extern "C" {
 
 const char* pfb_last_error(void) { return g_err; }

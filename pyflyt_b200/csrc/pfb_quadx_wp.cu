@@ -9,6 +9,7 @@
 // the grid reset the envs that finished on the previous launch (NEXT_STEP autoreset, inline warm-up).
 #include "pfb_noise.cuh"
 #include "pfb_quadx.cuh"
+#include "pfb_tail_reset.cuh"
 
 using namespace pfb;
 
@@ -157,10 +158,10 @@ __device__ __forceinline__ void qw_reset_env(const QuadXParams& p, const QxWaypo
   (void)qw_update_distance(w, s, wp);  // end_reset -> compute_state
 }
 
-// ---- spare post-reset states: the QuadX-Hover reset pipeline (pfb_lib.cu, DESIGN.md §4) for this env.  A spare is an
-// env-major record of 128 floats: the QW_* state words INCLUDING the episode's targets, new_distance and yaw error, then:
-enum { QSP_POSE = QW_ROWS, QSP_VALID = QW_ROWS + 6, QSP_FLAGS = QW_ROWS + 7, QSP_EPISODE = QW_ROWS + 8, QSP_ROWS = 128 };
-static_assert(QW_ROWS + 9 <= QSP_ROWS, "spare record too small");
+// spare post-reset states (pfb_tail_reset.cuh): an env-major record of 128 floats, the QW_* state words INCLUDING the
+// episode's targets, new_distance and yaw error, then the spare header
+enum { QSP_ROWS = 128 };
+static_assert(SpareHdr<QW_ROWS>::END <= QSP_ROWS, "spare record too small");
 int qwp_spare_rows() { return QSP_ROWS; }
 
 template <int MODE, bool INJECT, bool RANDACT, bool AUTORESET>
@@ -169,30 +170,18 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks)
                 const __grid_constant__ RngParams rng, float* __restrict__ st, int32_t* __restrict__ ist, float* __restrict__ actions,
                 const float* __restrict__ noise, float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ term,
                 uint8_t* __restrict__ trunc, uint8_t* __restrict__ info, const float* __restrict__ start_pos,
-                const float* __restrict__ start_orn, const int32_t* __restrict__ prev_count, const int32_t* __restrict__ prev_list,
-                int32_t* __restrict__ cur_count, int32_t* __restrict__ cur_list, int32_t* __restrict__ next_count,
-                float* __restrict__ spare, int spare_copy, int build, int tail_blocks, uint32_t step_seq, int64_t N) {
+                const float* __restrict__ start_orn, float* __restrict__ spare, const __grid_constant__ TailArgs a, int64_t N) {
   __shared__ float smem[kBlock * kQwObsStride];
   __shared__ uint8_t row_skip[kBlock];
   const int O = (h.angle_representation == 0 ? 20 : 21) + (w.use_yaw_targets ? 4 : 3) * w.num_targets;
-  const bool tail = AUTORESET && (int)blockIdx.x < tail_blocks;
-  const int64_t block_first = tail ? 0 : (int64_t)((int)blockIdx.x - (AUTORESET ? tail_blocks : 0)) * kBlock;
-  int t, t_end, t_stride;
-  if (tail) {
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !build) *next_count = 0;
-    t = blockIdx.x * kBlock + threadIdx.x;
-    t_end = prev_list ? *prev_count : (int)N;  // build mode after a user reset: every env
-    t_stride = tail_blocks * kBlock;
-  } else {
-    t = 0;
-    t_end = (block_first + threadIdx.x < N) ? 1 : 0;
-    t_stride = 1;
-  }
+  const uint32_t step_seq = a.step_seq;
+  TailWork sch = tail_schedule<1, AUTORESET>(a, N, threadIdx.x);
+  const bool tail = sch.tail;
   bool skip = true;
   float* row = smem + threadIdx.x * kQwObsStride;
 #pragma unroll 1
-  for (; t < t_end; t += t_stride) {
-    const int64_t i = tail ? (prev_list ? (int64_t)prev_list[t] : (int64_t)t) : block_first + threadIdx.x;
+  for (; sch.t < sch.t_end; sch.t += sch.t_stride) {
+    const int64_t i = tail_env<1>(a, sch, 0);
     QuadXRegs s;
     QwState wp;
     float act[4] = {0.f, 0.f, 0.f, 0.f};
@@ -204,20 +193,13 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks)
       // env.reset(): normally a copy of the env's spare (state, targets, distances of the NEXT episode); build mode
       // computes that spare; without a usable spare the warm-up runs inline with the same episode number
       float* rec = spare ? spare + i * QSP_ROWS : nullptr;
-      uint32_t nseq = step_seq | 0x40000000u;
-      bool hit = false;
       float pose[6];
 #pragma unroll
       for (int k = 0; k < 3; ++k) { pose[k] = start_pos[3 * i + k]; pose[3 + k] = start_orn[3 * i + k]; }
-      if (rec) {
-        nseq = __float_as_uint(rec[QSP_EPISODE]) + (build ? 1u : 0u);
-        hit = !build && spare_copy && rec[QSP_VALID] != 0.0f;
-#pragma unroll
-        for (int k = 0; k < 6; ++k) hit = hit && (rec[QSP_POSE + k] == pose[k]);
-      }
-      if (hit) {
+      const SpareProbe sp = spare_probe<QW_ROWS>(a, rec, pose, true);
+      if (sp.hit) {
         quadx_load<MODE>(rec, ist, N, i, s, 1, 0);
-        s.flags = __float_as_uint(rec[QSP_FLAGS]);
+        s.flags = __float_as_uint(rec[SpareHdr<QW_ROWS>::FLAGS]);
 #pragma unroll
         for (int k = 0; k < 4; ++k) { s.sp[k] = 0.0f; s.pwm[k] = rec[QX_PWM + k]; }
         for (int k = 0; k < 4 * w.num_targets; ++k) tb[(int64_t)(QW_TARGETS + k) * ts] = rec[QW_TARGETS + k];
@@ -226,28 +208,24 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks)
         wp.new_dist = rec[QW_DIST];
         wp.yaw_err = rec[QW_YAWERR];
       } else {
-        if (build) {
-          rec[QSP_VALID] = 0.0f;  // invalid until the warm-up below is stored
-#pragma unroll
-          for (int k = 0; k < 6; ++k) rec[QSP_POSE + k] = pose[k];
+        if (a.build) {
+          spare_open<QW_ROWS>(rec, pose);
           tb = rec;
           ts = 1;
         }
-        qw_reset_env<MODE, false>(p, w, rng, pose, nullptr, nullptr, nseq, N, i, tb, ts, s, wp);
+        qw_reset_env<MODE, false>(p, w, rng, pose, nullptr, nullptr, sp.episode, N, i, tb, ts, s, wp);
       }
-      if (build) {
+      if (a.build) {
         quadx_store<MODE>(rec, ist, N, i, s, false, 1, 0);
         rec[QW_DIST] = wp.new_dist;
         rec[QW_YAWERR] = wp.yaw_err;
-        rec[QSP_FLAGS] = __uint_as_float(s.flags);
-        rec[QSP_EPISODE] = __uint_as_float(nseq);
-        rec[QSP_VALID] = 1.0f;
+        spare_seal<QW_ROWS>(rec, s.flags, sp.episode);
         continue;
       }
       s.flags |= fresh_tag(step_seq);
     } else {
       quadx_load<MODE>(st, ist, N, i, s);
-      if (AUTORESET && (s.flags & (FLAG_TERM | FLAG_TRUNC | fresh_tag(step_seq)))) continue;  // a tail CTA owns this env
+      if (AUTORESET && tail_owns(s.flags, FLAG_TERM | FLAG_TRUNC, step_seq)) continue;
       s.flags &= ~(uint32_t)FLAG_FRESH_ANY;
       if (RANDACT) {  // uniform in the action box (quadx_base_env.py:79-102)
         uint64_t g = ((uint64_t)rng.env_offset_hi << 32 | rng.env_offset_lo) + (uint64_t)i;
@@ -302,34 +280,11 @@ __global__ void __launch_bounds__(kBlock, kMinBlocks)
       for (int k = 0; k < O; ++k) dst[k] = row[k];
     } else {
       skip = false;
-      if (AUTORESET) {
-        bool done = (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0;
-        unsigned m = __ballot_sync(__activemask(), done);
-        if (done) {
-          int lane = threadIdx.x & 31;
-          int leader = __ffs(m) - 1;
-          int base = 0;
-          if (lane == leader) base = atomicAdd(cur_count, __popc(m));
-          base = __shfl_sync(m, base, leader);
-          cur_list[base + __popc(m & ((1u << lane) - 1u))] = (int32_t)i;
-        }
-      }
+      if (AUTORESET) append_done(a, sch, __activemask(), (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0, i);
     }
   }
   if (tail) return;
-  row_skip[threadIdx.x] = skip ? 1 : 0;
-  __syncthreads();
-  int64_t rows = N - block_first;
-  if (rows > kBlock) rows = kBlock;
-  const int total = (int)rows * O;
-  float* dst = obs + block_first * O;
-  const int dr = kBlock / O, dc = kBlock - dr * O;
-  int r = threadIdx.x / O, c = threadIdx.x - r * O;
-  for (int j = threadIdx.x; j < total; j += kBlock) {
-    if (!row_skip[r]) dst[j] = smem[r * kQwObsStride + c];
-    r += dr; c += dc;
-    if (c >= O) { c -= O; ++r; }
-  }
+  flush_obs_tile<kQwObsStride>(smem, row_skip, skip, obs, sch, O, N);
 }
 
 template <int MODE, bool INJECT>
@@ -362,81 +317,32 @@ __global__ void __launch_bounds__(kBlock)
 // ---------------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------------
-#define QW_MODE_SWITCH(mode, BODY)                          \
-  switch (mode) {                                           \
-    case -1: { constexpr int MODE = -1; BODY; } break;      \
-    case 0: { constexpr int MODE = 0; BODY; } break;        \
-    case 1: { constexpr int MODE = 1; BODY; } break;        \
-    case 2: { constexpr int MODE = 2; BODY; } break;        \
-    case 3: { constexpr int MODE = 3; BODY; } break;        \
-    case 4: { constexpr int MODE = 4; BODY; } break;        \
-    case 5: { constexpr int MODE = 5; BODY; } break;        \
-    case 6: { constexpr int MODE = 6; BODY; } break;        \
-    case 7: { constexpr int MODE = 7; BODY; } break;        \
-    default: return fail("`mode` must be between -1 and 7, got %d", mode); \
-  }
+// k_qxwp_step for tail_env_step / tail_env_reset
+static auto qwp_step_launch(PfbContext* h, float* actions, const float* noise) {
+  return [=](auto inject, auto randact, auto autoreset, int grid, cudaStream_t s, float* spare, const TailArgs& a) -> int {
+    PFB_MODE_SWITCH(h->hover.flight_mode,
+                    (k_qxwp_step<MODE, decltype(inject)::value, decltype(randact)::value, decltype(autoreset)::value><<<grid, kBlock, 0, s>>>(
+                        h->qx, h->hover, h->qwp, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term,
+                        h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn, spare, a, h->n)));
+    return 0;
+  };
+}
 
 int qwp_env_reset(PfbContext* h, const uint8_t* mask, const float* noise, cudaStream_t s) {
-  const uint32_t seq = 0x80000000u | (uint32_t)h->reset_seq++;
   const int mode = h->hover.flight_mode;
-  const int g = grid_for(h->n);
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  if (spare) {
-    SPARE_BEFORE_RESET(h, s);
-    if (!mask) CUDA_OK(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(int32_t), s));  // a full reset empties the autoreset queues
-    else if (pfb_drop_masked_done(h, mask, s)) return -1;  // a masked one takes its envs out of the pending done list
-  }
+  auto reset = [&](uint32_t seq, int g) -> int {
 #define QR_ARGS h->qx, h->hover, h->qwp, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, h->buf.reset_targets, mask, noise, \
                 h->buf.obs, seq, h->n
-  if (noise) { QW_MODE_SWITCH(mode, (k_qxwp_reset<MODE, true><<<g, kBlock, 0, s>>>(QR_ARGS))); }
-  else { QW_MODE_SWITCH(mode, (k_qxwp_reset<MODE, false><<<g, kBlock, 0, s>>>(QR_ARGS))); }
+    if (noise) { PFB_MODE_SWITCH(mode, (k_qxwp_reset<MODE, true><<<g, kBlock, 0, s>>>(QR_ARGS))); }
+    else { PFB_MODE_SWITCH(mode, (k_qxwp_reset<MODE, false><<<g, kBlock, 0, s>>>(QR_ARGS))); }
 #undef QR_ARGS
-  LAUNCH_CHECK(h);
-  if (spare) {  // every env gets a fresh spare: the step kernel in build mode over all envs, same stream
-    QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, false, true><<<g, kBlock, 0, s>>>(
-                             h->qx, h->hover, h->qwp, h->rng, h->buf.state, h->buf.istate, h->buf.setpoint, nullptr, h->buf.obs, h->buf.reward,
-                             h->buf.term, h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn, nullptr, nullptr, nullptr, nullptr,
-                             nullptr, spare, 0, 1, g, 0u, h->n)));
-    LAUNCH_CHECK(h);
-  }
-  h->mode = mode;
+    return 0;
+  };
+  if (tail_env_reset(h, mask, s, reset, qwp_step_launch(h, h->buf.setpoint, nullptr))) return -1;
+  h->mode = mode;  // the env's flight mode, not the Aviary default
   return 0;
 }
 
 int qwp_env_step(PfbContext* h, float* actions, const float* noise, bool randact, cudaStream_t s) {
-  StepPlan pl = plan_step(h);
-  const int mode = h->hover.flight_mode;
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  const int spare_copy = (spare && !h->env.inline_reset) ? 1 : 0;
-  SPARE_BEFORE_STEP(h, s);
-  if (pl.prof) CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n], s));
-#define QS_ARGS h->qx, h->hover, h->qwp, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term,     \
-                h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, \
-                pl.cnt_next, spare, spare_copy, 0, pl.tail, pl.seq, h->n
-  if (h->env.autoreset) {
-    if (noise) return fail("injected noise (parity mode) is only supported with autoreset = 0");
-    if (randact) { QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, true, true><<<pl.grid, kBlock, 0, s>>>(QS_ARGS))); }
-    else { QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, false, true><<<pl.grid, kBlock, 0, s>>>(QS_ARGS))); }
-  } else {
-    if (noise) { QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, true, false, false><<<pl.grid, kBlock, 0, s>>>(QS_ARGS))); }
-    else if (randact) { QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, true, false><<<pl.grid, kBlock, 0, s>>>(QS_ARGS))); }
-    else { QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, false, false><<<pl.grid, kBlock, 0, s>>>(QS_ARGS))); }
-  }
-#undef QS_ARGS
-  LAUNCH_CHECK(h);
-  if (pl.prof) {
-    CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n + 1], s));
-    h->prof_n += 1;
-  }
-  if (spare) {  // rebuild the spares this launch consumed, on the side stream, while the next launches run
-    SPARE_REBUILD_BEGIN(h, s);
-    QW_MODE_SWITCH(mode, (k_qxwp_step<MODE, false, false, true><<<h->sm_count, kBlock, 0, h->side>>>(
-                             h->qx, h->hover, h->qwp, h->rng, h->buf.state, h->buf.istate, actions, nullptr, h->buf.obs, h->buf.reward, h->buf.term,
-                             h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur,
-                             pl.cnt_next, spare, 0, 1, h->sm_count, pl.seq, h->n)));
-    LAUNCH_CHECK(h);
-    SPARE_REBUILD_DONE(h);
-  }
-  h->step_seq += 1;
-  return 0;
+  return tail_env_step(h, noise, randact, s, qwp_step_launch(h, actions, noise));
 }

@@ -4,6 +4,7 @@
 
 #include "pfb_context.h"
 #include "pfb_noise.cuh"
+#include "pfb_tail_reset.cuh"
 #include "pfb_rocket_host.h"
 
 using namespace pfb;
@@ -196,10 +197,9 @@ static __device__ __noinline__ RocketRegs landing_reset_env_shared(const RocketP
 // whole register file instead of spilling (contact response + wind + variable-mass composite: ~170 live registers)
 constexpr int kLandBlocks = 8;
 
-// ---- spare post-reset states: the QuadX-Hover reset pipeline (pfb_lib.cu, DESIGN.md §4) for this env.  A spare is an
-// env-major record of 64 floats: the RK_* state words, then:
-enum { LSP_POSE = RK_ROWS, LSP_VALID = RK_ROWS + 6, LSP_FLAGS = RK_ROWS + 7, LSP_EPISODE = RK_ROWS + 8, LSP_ROWS = 64 };
-static_assert(RK_ROWS + 9 <= LSP_ROWS, "spare record too small");
+// spare post-reset states (pfb_tail_reset.cuh): an env-major record of 64 floats, the RK_* state words, then the spare header
+enum { LSP_ROWS = 64 };
+static_assert(SpareHdr<RK_ROWS>::END <= LSP_ROWS, "spare record too small");
 
 template <bool INJECT, bool RANDACT, bool AUTORESET>
 __global__ void __launch_bounds__(kBlock, kLandBlocks)
@@ -207,30 +207,18 @@ __global__ void __launch_bounds__(kBlock, kLandBlocks)
                 float* __restrict__ st, int32_t* __restrict__ ist, float* __restrict__ actions, const float* __restrict__ noise,
                 float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ term, uint8_t* __restrict__ trunc,
                 uint8_t* __restrict__ info, const float* __restrict__ start_pos, const float* __restrict__ start_orn,
-                const int32_t* __restrict__ prev_count, const int32_t* __restrict__ prev_list, int32_t* __restrict__ cur_count,
-                int32_t* __restrict__ cur_list, int32_t* __restrict__ next_count, float* __restrict__ spare, int spare_copy, int build,
-                int tail_blocks, uint32_t step_seq, int64_t N) {
+                float* __restrict__ spare, const __grid_constant__ TailArgs a, int64_t N) {
   __shared__ float smem[kBlock * kLandObsStride];
   __shared__ uint8_t row_skip[kBlock];
   const int O = (l.angle_representation == 0 ? 12 : 13) + 17;
-  const bool tail = AUTORESET && (int)blockIdx.x < tail_blocks;
-  const int64_t block_first = tail ? 0 : (int64_t)((int)blockIdx.x - (AUTORESET ? tail_blocks : 0)) * kBlock;
-  int t, t_end, t_stride;
-  if (tail) {
-    if (blockIdx.x == 0 && threadIdx.x == 0 && !build) *next_count = 0;
-    t = blockIdx.x * kBlock + threadIdx.x;
-    t_end = prev_list ? *prev_count : (int)N;  // build mode after a user reset: every env
-    t_stride = tail_blocks * kBlock;
-  } else {
-    t = 0;
-    t_end = (block_first + threadIdx.x < N) ? 1 : 0;
-    t_stride = 1;
-  }
+  const uint32_t step_seq = a.step_seq;
+  TailWork sch = tail_schedule<1, AUTORESET>(a, N, threadIdx.x);
+  const bool tail = sch.tail;
   bool skip = true;
   float* row = smem + threadIdx.x * kLandObsStride;
 #pragma unroll 1
-  for (; t < t_end; t += t_stride) {
-    const int64_t i = tail ? (prev_list ? (int64_t)prev_list[t] : (int64_t)t) : block_first + threadIdx.x;
+  for (; sch.t < sch.t_end; sch.t += sch.t_stride) {
+    const int64_t i = tail_env<1>(a, sch, 0);
     RocketRegs s;
     float act[7] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     int step_count = 0;
@@ -240,41 +228,26 @@ __global__ void __launch_bounds__(kBlock, kLandBlocks)
       // env.reset(): normally a copy of the env's spare; build mode computes that spare; without a usable spare the
       // warm-up runs inline with the same episode number (which also keys a randomised drop)
       float* rec = spare ? spare + i * LSP_ROWS : nullptr;
-      uint32_t nseq = step_seq | 0x40000000u;
-      bool hit = false;
       float pose[6];
 #pragma unroll
       for (int k = 0; k < 3; ++k) { pose[k] = start_pos[3 * i + k]; pose[3 + k] = start_orn[3 * i + k]; }
-      if (rec) {
-        nseq = __float_as_uint(rec[LSP_EPISODE]) + (build ? 1u : 0u);
-        hit = !build && spare_copy && rec[LSP_VALID] != 0.0f;
-        if (!l.randomize_drop) {  // a randomised drop does not read the start pose
-#pragma unroll
-          for (int k = 0; k < 6; ++k) hit = hit && (rec[LSP_POSE + k] == pose[k]);
-        }
-      }
-      if (hit) {
+      const SpareProbe sp = spare_probe<RK_ROWS>(a, rec, pose, !l.randomize_drop);  // a randomised drop does not read the start pose
+      if (sp.hit) {
         rocket_load(rec, ist, N, i, s, 1, 0);
-        s.flags = __float_as_uint(rec[LSP_FLAGS]);
+        s.flags = __float_as_uint(rec[SpareHdr<RK_ROWS>::FLAGS]);
       } else {
-        if (build) {
-          rec[LSP_VALID] = 0.0f;  // invalid until the warm-up below is stored
-#pragma unroll
-          for (int k = 0; k < 6; ++k) rec[LSP_POSE + k] = pose[k];
-        }
-        s = landing_reset_env_shared(&p, &l, &rng, pose[0], pose[1], pose[2], pose[3], pose[4], pose[5], nseq, l.randomize_drop, N, i);
+        if (a.build) spare_open<RK_ROWS>(rec, pose);
+        s = landing_reset_env_shared(&p, &l, &rng, pose[0], pose[1], pose[2], pose[3], pose[4], pose[5], sp.episode, l.randomize_drop, N, i);
       }
-      if (build) {
+      if (a.build) {
         rocket_store(rec, ist, N, i, s, false, 1, 0);
-        rec[LSP_FLAGS] = __uint_as_float(s.flags);
-        rec[LSP_EPISODE] = __uint_as_float(nseq);
-        rec[LSP_VALID] = 1.0f;
+        spare_seal<RK_ROWS>(rec, s.flags, sp.episode);
         continue;
       }
       s.flags |= fresh_tag(step_seq);
     } else {
       rocket_load(st, ist, N, i, s);
-      if (AUTORESET && (s.flags & (FLAG_TERM | FLAG_TRUNC | fresh_tag(step_seq)))) continue;  // a tail CTA owns this env
+      if (AUTORESET && tail_owns(s.flags, FLAG_TERM | FLAG_TRUNC, step_seq)) continue;
       s.flags &= ~(uint32_t)FLAG_FRESH_ANY;
       if (RANDACT) {  // rocket_base_env.py:82-107: [-1,1]^3, ignition {0..1}, throttle [0,1], gimbal [-1,1]^2
         uint64_t g = ((uint64_t)rng.env_offset_hi << 32 | rng.env_offset_lo) + (uint64_t)i;
@@ -320,34 +293,11 @@ __global__ void __launch_bounds__(kBlock, kLandBlocks)
       for (int k = 0; k < O; ++k) dst[k] = row[k];
     } else {
       skip = false;
-      if (AUTORESET) {
-        bool done = (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0;
-        unsigned m = __ballot_sync(__activemask(), done);
-        if (done) {
-          int lane = threadIdx.x & 31;
-          int leader = __ffs(m) - 1;
-          int base = 0;
-          if (lane == leader) base = atomicAdd(cur_count, __popc(m));
-          base = __shfl_sync(m, base, leader);
-          cur_list[base + __popc(m & ((1u << lane) - 1u))] = (int32_t)i;
-        }
-      }
+      if (AUTORESET) append_done(a, sch, __activemask(), (s.flags & (FLAG_TERM | FLAG_TRUNC)) != 0, i);
     }
   }
   if (tail) return;
-  row_skip[threadIdx.x] = skip ? 1 : 0;
-  __syncthreads();
-  int64_t rows = N - block_first;
-  if (rows > kBlock) rows = kBlock;
-  const int total = (int)rows * O;
-  float* dst = obs + block_first * O;
-  const int dr = kBlock / O, dc = kBlock - dr * O;
-  int r = threadIdx.x / O, c = threadIdx.x - r * O;
-  for (int j = threadIdx.x; j < total; j += kBlock) {
-    if (!row_skip[r]) dst[j] = smem[r * kLandObsStride + c];
-    r += dr; c += dc;
-    if (c >= O) { c -= O; ++r; }
-  }
+  flush_obs_tile<kLandObsStride>(smem, row_skip, skip, obs, sch, O, N);
 }
 
 template <bool INJECT>
@@ -412,67 +362,31 @@ int rk_observe(PfbContext* h, cudaStream_t s) {
   return 0;
 }
 
+// k_land_step for tail_env_step / tail_env_reset
+static auto rk_step_launch(PfbContext* h, float* actions, const float* noise) {
+  return [=](auto inject, auto randact, auto autoreset, int grid, cudaStream_t s, float* spare, const TailArgs& a) -> int {
+    k_land_step<decltype(inject)::value, decltype(randact)::value, decltype(autoreset)::value><<<grid, kBlock, 0, s>>>(
+        h->rk, h->land, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info,
+        h->buf.start_pos, h->buf.start_orn, spare, a, h->n);
+    return 0;
+  };
+}
+
 int rk_env_reset(PfbContext* h, const uint8_t* mask, const float* noise, cudaStream_t s) {
-  const uint32_t seq = 0x80000000u | (uint32_t)h->reset_seq++;
-  const int g = grid_for(h->n);
   // an explicit env.reset() honours the bound start_pos / start_orn unless randomize_drop is configured
   const int randomize = h->land.randomize_drop;
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  if (spare) {
-    SPARE_BEFORE_RESET(h, s);
-    if (!mask) CUDA_OK(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(int32_t), s));  // a full reset empties the autoreset queues
-    else if (pfb_drop_masked_done(h, mask, s)) return -1;  // a masked one takes its envs out of the pending done list
-  }
-  if (noise)
-    k_land_reset<true><<<g, kBlock, 0, s>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, mask, noise,
-                                            h->buf.obs, seq, randomize, h->n);
-  else
-    k_land_reset<false><<<g, kBlock, 0, s>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, mask,
-                                             nullptr, h->buf.obs, seq, randomize, h->n);
-  LAUNCH_CHECK(h);
-  if (spare) {  // every env gets a fresh spare: the step kernel in build mode over all envs, same stream
-    k_land_step<false, false, true><<<g, kBlock, 0, s>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, h->buf.setpoint, nullptr, h->buf.obs,
-                                                         h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info, h->buf.start_pos, h->buf.start_orn,
-                                                         nullptr, nullptr, nullptr, nullptr, nullptr, spare, 0, 1, g, 0u, h->n);
-    LAUNCH_CHECK(h);
-  }
-  h->mode = 0;
-  return 0;
+  auto reset = [&](uint32_t seq, int g) -> int {
+    if (noise)
+      k_land_reset<true><<<g, kBlock, 0, s>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, mask, noise,
+                                              h->buf.obs, seq, randomize, h->n);
+    else
+      k_land_reset<false><<<g, kBlock, 0, s>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, h->buf.start_pos, h->buf.start_orn, mask,
+                                               nullptr, h->buf.obs, seq, randomize, h->n);
+    return 0;
+  };
+  return tail_env_reset(h, mask, s, reset, rk_step_launch(h, h->buf.setpoint, nullptr));
 }
 
 int rk_env_step(PfbContext* h, float* actions, const float* noise, bool randact, cudaStream_t s) {
-  StepPlan pl = plan_step(h);
-  float* spare = h->env.autoreset ? h->d_spare : nullptr;
-  const int spare_copy = (spare && !h->env.inline_reset) ? 1 : 0;
-  SPARE_BEFORE_STEP(h, s);
-  if (pl.prof) CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n], s));
-#define LD_ARGS h->rk, h->land, h->rng, h->buf.state, h->buf.istate, actions, noise, h->buf.obs, h->buf.reward, h->buf.term, h->buf.trunc, \
-                h->buf.info, h->buf.start_pos, h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, pl.cnt_next, spare, \
-                spare_copy, 0, pl.tail, pl.seq, h->n
-  if (h->env.autoreset) {
-    if (noise) return fail("injected noise (parity mode) is only supported with autoreset = 0");
-    if (randact) k_land_step<false, true, true><<<pl.grid, kBlock, 0, s>>>(LD_ARGS);
-    else k_land_step<false, false, true><<<pl.grid, kBlock, 0, s>>>(LD_ARGS);
-  } else {
-    if (noise) k_land_step<true, false, false><<<pl.grid, kBlock, 0, s>>>(LD_ARGS);
-    else if (randact) k_land_step<false, true, false><<<pl.grid, kBlock, 0, s>>>(LD_ARGS);
-    else k_land_step<false, false, false><<<pl.grid, kBlock, 0, s>>>(LD_ARGS);
-  }
-#undef LD_ARGS
-  LAUNCH_CHECK(h);
-  if (pl.prof) {
-    CUDA_OK(cudaEventRecord(h->prof_ev[2 * h->prof_n + 1], s));
-    h->prof_n += 1;
-  }
-  if (spare) {  // rebuild the spares this launch consumed, on the side stream, while the next launches run
-    SPARE_REBUILD_BEGIN(h, s);
-    k_land_step<false, false, true><<<h->sm_count, kBlock, 0, h->side>>>(h->rk, h->land, h->rng, h->buf.state, h->buf.istate, actions, nullptr, h->buf.obs,
-                                                                         h->buf.reward, h->buf.term, h->buf.trunc, h->buf.info, h->buf.start_pos,
-                                                                         h->buf.start_orn, pl.cnt_prev, pl.list_prev, pl.cnt_cur, pl.list_cur, pl.cnt_next,
-                                                                         spare, 0, 1, h->sm_count, pl.seq, h->n);
-    LAUNCH_CHECK(h);
-    SPARE_REBUILD_DONE(h);
-  }
-  h->step_seq += 1;
-  return 0;
+  return tail_env_step(h, noise, randact, s, rk_step_launch(h, actions, noise));
 }
